@@ -15,6 +15,9 @@ each with its own roofline fraction, CPU baseline and parity check against the C
   python bench.py --gpus 1 --steps 20 --warmup 3            # our arm (CUDA kernels through the C ABI)
   python bench.py --impl reference --steps 3 --warmup 1     # reference arm: CPU restatement on all host cores
   torchrun ... bench.py --gpus N ...                        # one rank per GPU, shards range-partitioned, merged count
+  python bench.py --steps 20 --dump-outputs DIR             # also DIR/<name>.npy: what each timed query returned in its last step
+
+The inputs are generated from fixed seeds, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -28,6 +31,10 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True       # the tree may be read-only where the benchmark runs: leave no __pycache__ in it
+
+# name -> what a timed query returned to its caller in its last timed step (merged over ranks); --dump-outputs writes them
+LAST_OUTPUTS = {}
 
 FIELD_SEED_ID = 1
 ROWS_A, ROWS_B = list(range(32)), list(range(32, 64))
@@ -207,6 +214,9 @@ def run_reference(args):
                        "ms": psec * 1e3, "set_ops_per_sec": len(PAIRS_A) * S / psec},
         "check_count": count,
     }
+    if args.dump_outputs:
+        LAST_OUTPUTS["headline_count"] = np.array([count], dtype=np.uint64)
+        dump_outputs(args.dump_outputs)
     print(json.dumps(line))
     return 0
 
@@ -224,7 +234,7 @@ def timed_calls(ctx, fn, steps, warmup):
     return float(np.mean(ms)), float(np.min(ms)), wall
 
 
-def pair_record(h, idx, fld, shards, rows_a, rows_b, label, cpu, frags, peak, world, dist, torch, steps):
+def pair_record(h, idx, fld, shards, rows_a, rows_b, label, name, cpu, frags, peak, world, dist, torch, steps):
     """Count(Intersect(Row a_k, Row b_k)) over this rank's shards: (i) one query per launch, rotating over the row pairs, (ii) all pairs
     fused in one launch (SURVEY §8d).  Parity of every pair's count against the CPU port over ALL shards (all ranks)."""
     from featurebase_b200 import executor as X, lib as L
@@ -255,6 +265,7 @@ def pair_record(h, idx, fld, shards, rows_a, rows_b, label, cpu, frags, peak, wo
     algo_one = algo_all / n_pairs
     got = np.asarray(batched[0], dtype=np.uint64)
     got_single = np.array([single[k] for k in range(n_pairs)], dtype=np.uint64)
+    LAST_OUTPUTS[name + "_single"], LAST_OUTPUTS[name + "_batched"] = got_single, got
     names = ("absent", "array", "bitmap", "run")      # device-side analogue of the reference's statsHit("intersectionCount/...") counters
     hm = ctx.pair_types(idx.id, fld.id, 0, rows_a[0], fld.id, 0, rows_b[0], shards)
     hist = {"%s x %s" % (names[i], names[j]): int(hm[i][j]) for i in range(4) for j in range(4) if hm[i][j]}
@@ -294,7 +305,7 @@ def pair_record(h, idx, fld, shards, rows_a, rows_b, label, cpu, frags, peak, wo
 
 def north_star(h, idx, fld, shards, cpu, frags, peak, world, dist, torch, steps):
     """BASELINE configs[4] at its acceptance point (1 %, 1 B columns per GPU)"""
-    return pair_record(h, idx, fld, shards, PAIRS_A, PAIRS_B, "1 % density (uniform)", cpu, frags, peak, world, dist, torch, steps)
+    return pair_record(h, idx, fld, shards, PAIRS_A, PAIRS_B, "1 % density (uniform)", "north_star", cpu, frags, peak, world, dist, torch, steps)
 
 
 SWEEP_POINTS = [(0.0001, 0, 8), (0.001, 0, 8), (0.1, 0, 2), (0.5, 0, 2), (0.01, 1, 8), (0.2, 1, 2)]   # (density, generator mode, row pairs); 1 % uniform = north_star
@@ -315,7 +326,7 @@ def density_sweep(h, idx, rank, S, cpu, peak, world, dist, torch, steps):
         h.ctx.commit()
         frags = cpu.fragments(bulk, S) if cpu is not None else None
         label = "%g %% density (%s)" % (p * 100, "uniform" if mode == 0 else "clustered, mean run 64")
-        rec = pair_record(h, idx, fld, shards, rows[0::2], rows[1::2], label, cpu, frags, peak, world, dist, torch, max(steps // 2, 8))
+        rec = pair_record(h, idx, fld, shards, rows[0::2], rows[1::2], label, "density_sweep_%d" % k, cpu, frags, peak, world, dist, torch, max(steps // 2, 8))
         rec.update({"density": p, "generator": "uniform" if mode == 0 else "clustered"})
         out.append(rec)
         del bulk, frags
@@ -348,6 +359,7 @@ def config3(cpu, peak, steps, local):
         res[i % nf] = h.ctx.count(idx.id, progs[i % nf], shards)
 
     ms, ms_min, wall = timed_calls(h.ctx, step, max(steps, 4 * nf), nf)
+    LAST_OUTPUTS["config3_counts"] = np.array([res[k] for k in range(nf)], dtype=np.uint64)     # field k's last timed count
     pay, nc = h.ctx.rows_payload_bytes(idx.id, idx.fields["v0"].id, X.VIEW_BSI, shards, None)
     algo = pay + 16 * nc + 8
     rec = {"query": "Count(Row(v > 2^31)), 10,000,000 records, 32-bit int field", "kernel": "eval_wordpar_kernel", "ms": ms, "ms_min": ms_min, "e2e_ms": wall,
@@ -394,6 +406,7 @@ def config4(cpu, peak, steps, local, rank, world, dist, torch, uid_fn):
         res[0] = h.ctx.groupby(idx.id, [fa.id, fb.id], [0, 0], [rows, rows], shards)
 
     ms, ms_min, wall = timed_calls(h.ctx, step, max(steps, 10), 3)
+    LAST_OUTPUTS["config4_groupby"] = np.asarray(res[0])
     if world > 1:
         t = torch.tensor([ms, wall], device="cuda", dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -424,10 +437,18 @@ def config4(cpu, peak, steps, local, rank, world, dist, torch, uid_fn):
     return rec
 
 
+def dump_outputs(path):
+    """LAST_OUTPUTS as DIR/<name>.npy.  Every value is a count below 2^53, so float64 holds it exactly; all of them together
+    are under 1 MB."""
+    os.makedirs(path, exist_ok=True)
+    for name, arr in LAST_OUTPUTS.items():
+        np.save(os.path.join(path, name + ".npy"), np.asarray(arr, dtype=np.uint64).astype(np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps of the headline query")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours")
     ap.add_argument("--shards-per-gpu", type=int, default=1024)
@@ -437,7 +458,10 @@ def main():
     ap.add_argument("--extras", default="north_star,density_sweep,config3,config4", help="which sub-records to produce (comma list)")
     ap.add_argument("--reduce", default="p2p", choices=["p2p", "nccl"], help="N>1: fused peer-memory Count merge (default) or ncclAllReduce")
     ap.add_argument("--cold", action="store_true", help="also time fragment upload + query (e2e_cold_load)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what each timed query returned in its last timed step to DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
     if int(os.environ.get("LOCAL_RANK", "0")) == 0:
@@ -531,6 +555,7 @@ def main():
         assert got == expect
     sync_all()
     wall = time.perf_counter() - t_begin
+    LAST_OUTPUTS["headline_count"] = np.array([got], dtype=np.uint64)
     launches = h.ctx.counters()["kernel_launches"] - c0
     kms = float(np.mean(kernel_ms))
     # max over ranks (device time of the kernels; wall time of the C-ABI calls)
@@ -639,6 +664,8 @@ def main():
         if cold:
             line["e2e_cold_load"] = cold
         line.update(extras)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs)
         print(json.dumps(line))
     if world > 1:
         dist.barrier()

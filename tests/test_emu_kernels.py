@@ -169,13 +169,15 @@ def test_bench_main_runs_against_interpreted_library():
     assert d["check_count"] == exp > 0
 
 
-def test_bench_sub_records_run_against_interpreted_library():
+def test_bench_sub_records_run_against_interpreted_library(tmp_path):
     """bench.py's north_star and density_sweep sub-records on 4 shards, CPU port included: every point's parity_ok (GPU arm's counts,
-    single and batched, against the CPU port over all shards) must hold — these are the checks the driver sees at full size"""
+    single and batched, against the CPU port over all shards) must hold — these are the checks bench.py reports at full size.
+    --dump-outputs writes the same counts as .npy files."""
     import json
+    import numpy as np
     e = dict(os.environ, FBGPU_LIB=emu_lib())
-    r = subprocess.run([sys.executable, os.path.join(EMU, "bench_shim.py"), "--steps", "2", "--warmup", "1", "--shards-per-gpu", "4", "--extras", "north_star,density_sweep"],
-                       cwd=ROOT, env=e, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=1500)
+    r = subprocess.run([sys.executable, os.path.join(EMU, "bench_shim.py"), "--steps", "2", "--warmup", "1", "--shards-per-gpu", "4", "--extras", "north_star,density_sweep",
+                        "--dump-outputs", str(tmp_path)], cwd=ROOT, env=e, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=1500)
     assert r.returncode == 0, r.stderr[-2000:]
     d = json.loads(r.stdout.strip().splitlines()[-1])
     assert d["parity_ok"] is True and d["north_star"]["parity_ok"] is True and d["north_star"]["counts_sum"] > 0
@@ -185,6 +187,14 @@ def test_bench_sub_records_run_against_interpreted_library():
         assert rec["container_pair_types_pair0"] and "cpu_baseline" in rec
     kinds = set(k for rec in d["density_sweep"] for k in rec["container_pair_types_pair0"])
     assert {"array x array", "bitmap x bitmap"} <= kinds and any("run" in k for k in kinds), kinds
+    out = {p.stem: np.load(p) for p in tmp_path.glob("*.npy")}
+    names = {"headline_count"} | {"%s_%s" % (n, k) for n in ["north_star"] + ["density_sweep_%d" % i for i in range(6)] for k in ("single", "batched")}
+    assert set(out) == names and all(a.dtype == np.float64 for a in out.values())
+    assert out["headline_count"].tolist() == [d["check_count"]]
+    assert out["north_star_batched"].shape == (32,) and out["north_star_batched"].sum() == d["north_star"]["counts_sum"]
+    for i, rec in enumerate(d["density_sweep"]):
+        assert np.array_equal(out["density_sweep_%d_single" % i], out["density_sweep_%d_batched" % i])
+        assert out["density_sweep_%d_batched" % i].sum() == rec["counts_sum"]
 
 
 def test_bench_sweep_runs_against_interpreted_library():

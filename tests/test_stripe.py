@@ -17,9 +17,15 @@ def lib(tmp_path_factory):
     subprocess.check_call(["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-I", os.path.join(ROOT, "featurebase_b200", "csrc"),
                            os.path.join(ROOT, "tests", "native", "stripe_check.cpp"), "-o", out])
     L = C.CDLL(out)
-    L.wavefronts.restype = C.c_uint64
-    L.worst.restype = C.c_uint32
-    L.word_offset_mismatches.restype = C.c_uint64
+    # pointers must be declared: ctypes passes an undeclared Python int as a 32-bit C int
+    vp, u32 = C.c_void_p, C.c_uint32
+    L.stripe.argtypes = [vp, vp, u32]
+    L.wavefronts.argtypes, L.wavefronts.restype = [vp, u32], C.c_uint64
+    L.worst.argtypes, L.worst.restype = [vp, u32], C.c_uint32
+    L.word_offset_mismatches.argtypes, L.word_offset_mismatches.restype = [], C.c_uint64
+    L.load_array.argtypes = [vp, vp, u32, C.c_int]
+    L.model_scatter.argtypes = [C.c_int, vp, u32, vp]
+    L.model_probe.argtypes = [vp, u32, vp]
     return L
 
 
